@@ -5,7 +5,7 @@ A "step" = one body of GHRegistration::ghicp_reg's while-loop (src/ghicp_reg.cpp
 excluded): calED + calCD_* + findcorrespondence* + transformestimation + adjustweight.
 Default workload = BASELINE.json configs[1]: 50k x 50k keypoints, BSC descriptors, KM matching, 6-DoF.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for every field.
 """
@@ -185,6 +185,21 @@ NCU_TRAFFIC = {"config2": {"bytes": 5.038999e9 + 0.32185856e9,
                                "source": "profiles/r02_ncu_k_stream_nnr.raw.csv (ncu --set full, k_stream<1,1,1,1,1>, round 2)"},
                "config2-nn": {"bytes": 5.311e9, "source": "profiles/r01_summary.md (ncu --set full capture of k_stream NN, round 1)"}}
 
+DUMP_BYTES = 64 << 20   # --dump-outputs writes at most this much; a larger array is replaced by a seeded sample of its rows
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy (float64), rows sampled with a fixed seed where the whole would not fit."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > budget:
+            rows = budget // max(1, a.nbytes // max(1, len(a)))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), rows, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 FT = {"none": 3, "bsc": 0, "fpfh": 2}
 CT = {"nn": 0, "nnr": 1, "km": 2}
 
@@ -336,6 +351,8 @@ def _main(saved_stdout):
     ap.add_argument("--n", type=int, default=0, help="override N=M (e.g. 4000: a size the reference runs WITHOUT extrapolation)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="N=M of the CPU arm's main sample")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (pairs, keypoints, transforms, statistics) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3  # timing rule: >= 3 warm-up steps
@@ -505,6 +522,13 @@ def _main(saved_stdout):
     barrier()
     clocks = cs.summary()
     ms_per_step = allmax(wall * 1e3 / args.steps)
+    if args.dump_outputs and rank == 0:
+        sp, tp = reg.pairs()
+        dump_outputs(args.dump_outputs, {
+            "source_pairs": sp, "target_pairs": tp, "source_keypoints": reg.source(), "rt_step": st.Rt_np(),
+            "rt_accumulated": st.Rt_tillnow_np(),
+            "stats": [st.iteration, st.cor, st.converged, st.penalty, st.rmse, st.rmse_after, st.fdm, st.fdstd, st.iou, st.para1,
+                      st.para2, st.km_energy]})
 
     # ---- timed region 2: end to end through the host-facing API -----------------------------------
     # every step: host (pinned inside the library) -> device copy of the current source + target

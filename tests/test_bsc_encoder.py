@@ -1,6 +1,6 @@
 """BSC descriptor encoder (SURVEY.md §8f row N2) without a GPU:
-  * the oracle restatement (oracle/ghicp_bsc_oracle.cpp) against the reference's own header compiled verbatim
-    (oracle/_ref/libbsc_ref.so; only where /root/reference exists) and against the committed golden vectors made from it;
+  * the oracle restatement (oracle/ghicp_bsc_oracle.cpp) against the outputs of the reference's own header compiled
+    verbatim (oracle/_ref/libbsc_ref.so), stored in tests/golden/reference_golden.npz and tests/golden/bsc_golden.npz;
   * structural properties of the reference's descriptor (bit layout, the re-arranged variants' quirk, rigid invariance);
   * the product's kernel (k_bsc in gh-icp_b200/csrc/ghicp_prep.cu) run on the CPU through the host emulation shim, against
     the oracle.  TOLERANCE: the kernel holds exact sums where the reference accumulates in float32 in KD-tree order
@@ -13,6 +13,7 @@ import os
 import numpy as np
 import pytest
 
+import reference_golden as rg
 from test_prep_oracle import scan_like_cloud
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -62,18 +63,22 @@ def test_oracle_reproduces_the_golden_vectors_of_the_reference_build(orc, gold):
         assert b.shape[0] == V and np.array_equal(b, gold["bits"][:V])
 
 
-@pytest.mark.parametrize("n,nkp,radius,seed", [(3000, 40, 1.0, 1), (5000, 30, 0.6, 2), (1500, 25, 2.0, 3)])
-def test_oracle_equals_the_reference_build_on_fresh_scenes(orc, scratch_cwd, n, nkp, radius, seed):
-    if orc.ref_bsc_lib() is None:
-        pytest.skip("reference build not available (no /root/reference)")
-    pairs = orc.ref_bsc_pattern(7)
+FRESH_CASES = [(3000, 40, 1.0, 1), (5000, 30, 0.6, 2), (1500, 25, 2.0, 3)]
+
+
+def fresh_scene(n, nkp, seed):
     xyz = scan_like_cloud(n, seed, extent=(10.0, 10.0, 4.0))
-    kp = np.random.default_rng(seed).choice(n, nkp, replace=False).astype(np.int32)
+    return xyz, np.random.default_rng(seed).choice(n, nkp, replace=False).astype(np.int32)
+
+
+@pytest.mark.parametrize("n,nkp,radius,seed", FRESH_CASES)
+def test_oracle_equals_the_reference_build_on_fresh_scenes(orc, gold, n, nkp, radius, seed):
+    ref = rg.load(rg.key("bsc_fresh", n, nkp, radius, seed))
+    xyz, kp = fresh_scene(n, nkp, seed)
     for dof in (0, 4, 6):
-        ref_bits, ref_lrf = orc.ref_bsc_extract(xyz, kp, radius, pairs, 7, dof)
-        bits, lrf, _ = orc.bsc_extract(xyz, kp, radius, pairs, 7, dof)
-        assert np.array_equal(bits, ref_bits)
-        assert np.array_equal(lrf, ref_lrf)
+        bits, lrf, _ = orc.bsc_extract(xyz, kp, radius, gold["pairs"], 7, dof)
+        assert np.array_equal(rg.digest(bits), ref[f"dof{dof}/bits"])
+        assert np.array_equal(rg.digest(lrf), ref[f"dof{dof}/lrf"])
 
 
 def test_shipped_pattern_is_what_the_reference_constructor_generates(orc, scratch_cwd, gold):
@@ -223,50 +228,51 @@ def _degenerate_clouds():
     return {"plane": plane, "line": line, "duplicates": dup, "lattice": lattice, "tiny": tiny, "far": far}
 
 
+def degenerate_case(name, xyz):
+    """(radius, keypoints) of the degenerate cloud `name`."""
+    return {"tiny": 1e-3, "lattice": 0.9}.get(name, 1.0), np.arange(0, len(xyz), max(1, len(xyz) // 24), dtype=np.int32)
+
+
 @pytest.mark.parametrize("name", ["plane", "line", "duplicates", "lattice", "tiny", "far"])
-def test_oracle_equals_the_reference_build_on_degenerate_geometry(orc, scratch_cwd, name):
+def test_oracle_equals_the_reference_build_on_degenerate_geometry(orc, gold, name):
     """Zero and repeated eigenvalues, coincident points, symmetric lattices (masses of exactly equal distances: the tie order of
     the neighbour search matters), very small and very large coordinates."""
-    if orc.ref_bsc_lib() is None:
-        pytest.skip("reference build not available (no /root/reference)")
+    ref = rg.load(rg.key("bsc_degenerate", name))
     xyz = _degenerate_clouds()[name]
-    radius = {"tiny": 1e-3, "lattice": 0.9}.get(name, 1.0)
-    pairs = orc.ref_bsc_pattern(7)
-    kp = np.arange(0, len(xyz), max(1, len(xyz) // 24), dtype=np.int32)
+    radius, kp = degenerate_case(name, xyz)
     for dof in (0, 6):
-        ref_bits, ref_lrf = orc.ref_bsc_extract(xyz, kp, radius, pairs, 7, dof)
-        bits, lrf, status = orc.bsc_extract(xyz, kp, radius, pairs, 7, dof)
+        bits, lrf, status = orc.bsc_extract(xyz, kp, radius, gold["pairs"], 7, dof)
         assert status.sum() == 0
-        assert np.array_equal(bits, ref_bits), name
-        assert np.array_equal(lrf, ref_lrf, equal_nan=True), name
+        assert np.array_equal(rg.digest(bits), ref[f"dof{dof}/bits"]), name
+        assert np.array_equal(rg.digest(lrf), ref[f"dof{dof}/lrf"]), name                 # NaN equal to NaN
 
 
-def test_oracle_equals_the_reference_build_randomised(orc, scratch_cwd):
-    """Hypothesis-driven: random small clouds (uniform, clustered or layered), radii, keypoints, dof types."""
-    if orc.ref_bsc_lib() is None:
-        pytest.skip("reference build not available (no /root/reference)")
-    from hypothesis import given, settings, strategies as st, HealthCheck
-    pairs = orc.ref_bsc_pattern(7)
+RANDOM_CASES = 40
+RANDOM_KINDS = ["uniform", "clustered", "layered"]
 
-    @settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(seed=st.integers(0, 2 ** 31 - 1), n=st.integers(30, 500), kind=st.sampled_from(["uniform", "clustered", "layered"]),
-           radius=st.floats(0.2, 3.0), dof=st.sampled_from([0, 2, 4, 6]))
-    def run(seed, n, kind, radius, dof):
-        rng = np.random.default_rng(seed)
-        P = rng.random((n, 3)) * [5.0, 5.0, 2.0]
-        if kind == "clustered":
-            P = P[rng.integers(0, max(3, n // 20), n)] + 0.05 * rng.standard_normal((n, 3))
-        elif kind == "layered":
-            P[:, 2] = np.round(P[:, 2] * 2) / 2
-        xyz = P.astype(np.float32)
-        kp = rng.choice(n, min(n, 12), replace=False).astype(np.int32)
-        ref_bits, ref_lrf = orc.ref_bsc_extract(xyz, kp, radius, pairs, 7, dof)
-        bits, lrf, status = orc.bsc_extract(xyz, kp, radius, pairs, 7, dof)
+
+def random_scene(seed, n, kind):
+    rng = np.random.default_rng(seed)
+    P = rng.random((n, 3)) * [5.0, 5.0, 2.0]
+    if RANDOM_KINDS[kind] == "clustered":
+        P = P[rng.integers(0, max(3, n // 20), n)] + 0.05 * rng.standard_normal((n, 3))
+    elif RANDOM_KINDS[kind] == "layered":
+        P[:, 2] = np.round(P[:, 2] * 2) / 2
+    return P.astype(np.float32), rng.choice(n, min(n, 12), replace=False).astype(np.int32)
+
+
+def test_oracle_equals_the_reference_build_randomised(orc, gold):
+    """40 random small clouds (uniform, clustered or layered), radii, keypoints and dof types, drawn once from a fixed seed
+    (the parameters are stored with the reference's outputs)."""
+    params = rg.load("bsc_random")["params"]
+    assert len(params) == RANDOM_CASES
+    for i, (seed, n, kind, radius, dof) in enumerate(params):
+        ref = rg.load(rg.key("bsc_random", i))
+        xyz, kp = random_scene(int(seed), int(n), int(kind))
+        bits, lrf, status = orc.bsc_extract(xyz, kp, float(radius), gold["pairs"], 7, int(dof))
         ok = status == 0                      # < 3 neighbours: the reference reads uninitialised axes; not comparable
-        assert np.array_equal(bits[:, ok], ref_bits[:, ok])
-        assert np.array_equal(lrf[ok], ref_lrf[ok], equal_nan=True)
-
-    run()
+        assert np.array_equal(bits[:, ok], ref[f"dof{int(dof)}/bits"][:, ok]), i
+        assert np.array_equal(lrf[ok], ref[f"dof{int(dof)}/lrf"][ok], equal_nan=True), i
 
 
 @pytest.mark.parametrize("name", ["line", "duplicates", "tiny", "far", "plane"])

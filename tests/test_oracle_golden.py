@@ -1,6 +1,6 @@
 """Pins the CPU oracle against every golden vector the reference holds for the hot path
-(SURVEY.md §4: G1, G2, G4) and against the reference's own src/km.cpp compiled verbatim
-(oracle/_ref/libkm_ref.so), plus independent numpy/scipy cross-checks."""
+(SURVEY.md §4: G1, G2, G4) and against the stored outputs of the reference's own src/km.cpp compiled verbatim
+(oracle/_ref/libkm_ref.so, tests/golden/reference_golden.npz), plus independent numpy/scipy cross-checks."""
 import json
 import math
 import os
@@ -10,6 +10,7 @@ import pytest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
+import reference_golden as rg  # noqa: E402
 from golden_vectors import G1_W, G2_CD, G2_PAIRS  # noqa: E402
 
 
@@ -44,16 +45,18 @@ def test_golden_fixture_file_matches(orc, scratch_cwd):
         assert m.tolist() == case["match"], case["name"]
 
 
-@pytest.mark.parametrize("n,seed", [(8, 0), (40, 1), (150, 2), (300, 3)])
-def test_port_equals_reference_km_bitwise(orc, scratch_cwd, n, seed):
-    if orc.ref_km_lib() is None:
-        pytest.skip("oracle/_ref not built (reference absent)")
+KM_CASES = [(8, 0), (40, 1), (150, 2), (300, 3)]
+
+
+def km_case(orc, n, seed):
     rng = np.random.default_rng(seed)
-    CD = rng.random((n, n - n // 5)) * 60.0
-    G = orc.km_graph(CD, 25.0)
-    a = orc.km_solve(G, 0.01, "port")
-    b = orc.km_solve(G, 0.01, "ref")
-    assert np.array_equal(a, b)
+    return orc.km_graph(rng.random((n, n - n // 5)) * 60.0, 25.0)
+
+
+@pytest.mark.parametrize("n,seed", KM_CASES)
+def test_port_equals_reference_km_bitwise(orc, scratch_cwd, n, seed):
+    a = orc.km_solve(km_case(orc, n, seed), 0.01, "port")
+    assert np.array_equal(a, rg.load(rg.key("km", n, seed))["match"])
 
 
 @pytest.mark.parametrize("n,seed", [(30, 5), (120, 6)])
@@ -221,27 +224,33 @@ def test_oracle_fd_fpfh_equals_reference_fixture(orc):
     assert np.isnan(D[:, 12]).all() and D[10, 11] == pytest.approx(1.0, abs=1e-6)
 
 
-def test_reference_feature_code_live(orc):
-    """When /root/reference is present (build container): the oracle against the reference's own functions on fresh random
-    inputs, and the descriptor bit layout (setNthBitValue: bit k -> byte k/8, bit k%8) the synthetic generator assumes."""
-    R = orc.ref_feat_lib()
-    if R is None:
-        pytest.skip("oracle/_ref/libfeat_ref.so not built (no /root/reference here)")
-    import ctypes as C
-    import ghicp_b200 as g
+FEATURE_BITS = (441, 672, 13)
+
+
+def feature_code_inputs():
+    """Random descriptor pairs, bit sets and FPFH histogram pairs (fixed seed) the reference's feature code was run on."""
     rng = np.random.default_rng(5)
-    for bits in (441, 672, 13):
+    d = {}
+    for bits in FEATURE_BITS:
         B = (bits + 7) // 8
-        for _ in range(50):
-            a = rng.integers(0, 256, B, dtype=np.uint8); b = rng.integers(0, 256, B, dtype=np.uint8)
-            assert orc.hamming(a, b) == R.featref_hamming(a.ctypes.data, b.ctypes.data, bits)
-        bits01 = rng.random(bits) < 0.4
-        pos = np.nonzero(bits01)[0].astype(np.int32)
-        out = np.zeros(B, np.uint8)
-        R.featref_set_bits(bits, pos.ctypes.data_as(C.POINTER(C.c_int)), len(pos), out.ctypes.data)
-        assert np.array_equal(out, g.synth.pack_bits(bits01))
-        assert all(R.featref_get_bit(out.ctypes.data, bits, int(k)) == int(bits01[k]) for k in range(bits))
-    for _ in range(200):
-        h1 = (rng.gamma(0.6, 1.0, 33) * 20).astype(np.float32); h2 = (rng.gamma(0.6, 1.0, 33) * 20).astype(np.float32)
-        a = np.float32(orc.fpfh_distance(h1, h2)); b = np.float32(R.featref_fpfh_distance(h1.ctypes.data, h2.ctypes.data))
-        assert a == b
+        d[f"pairs{bits}"] = [(rng.integers(0, 256, B, dtype=np.uint8), rng.integers(0, 256, B, dtype=np.uint8)) for _ in range(50)]
+        d[f"bits{bits}"] = rng.random(bits) < 0.4
+    d["fpfh"] = [((rng.gamma(0.6, 1.0, 33) * 20).astype(np.float32), (rng.gamma(0.6, 1.0, 33) * 20).astype(np.float32))
+                 for _ in range(200)]
+    return d
+
+
+def test_reference_feature_code_live(orc):
+    """The oracle against the stored outputs of the reference's own functions (StereoBinaryFeature::hammingDistance,
+    setNthBitValue / getNthBitValue, compute_fpfh_distance) on random inputs, and the descriptor bit layout (setNthBitValue:
+    bit k -> byte k/8, bit k%8) the synthetic generator assumes."""
+    import ghicp_b200 as g
+    ref = rg.load("feat")
+    x = feature_code_inputs()
+    for bits in FEATURE_BITS:
+        assert [orc.hamming(a, b) for a, b in x[f"pairs{bits}"]] == ref[f"hamming{bits}"].tolist()
+        bits01 = x[f"bits{bits}"]
+        assert np.array_equal(ref[f"set_bits{bits}"], g.synth.pack_bits(bits01))
+        assert np.array_equal(ref[f"get_bit{bits}"], bits01.astype(np.int32))
+    a = np.array([orc.fpfh_distance(h1, h2) for h1, h2 in x["fpfh"]], np.float32)
+    assert np.array_equal(a, ref["fpfh_distance"])

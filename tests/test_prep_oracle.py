@@ -8,6 +8,8 @@ import subprocess
 import numpy as np
 import pytest
 
+import reference_golden as rg
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 fp, ip, dp = C.POINTER(C.c_float), C.POINTER(C.c_int), C.POINTER(C.c_double)
 
@@ -44,16 +46,18 @@ def test_voxel_filter_one_point_per_voxel_smallest_index_plus_phantom(orc):
     assert np.all(np.diff(key[rest]) > 0)
 
 
-@pytest.mark.parametrize("n,voxel,seed", [(6000, 0.4, 1), (20000, 0.1, 2), (500, 5.0, 3), (3000, 0.02, 4)])
+VOXEL_CASES = [(6000, 0.4, 1), (20000, 0.1, 2), (500, 5.0, 3), (3000, 0.02, 4)]
+KEYPOINT_CASES = [(4000, 1.0, 1.5, 8), (1500, 0.6, 0.6, 9), (600, 3.0, 0.3, 10), (6000, 0.8, 1.0, 12)]
+
+
+@pytest.mark.parametrize("n,voxel,seed", VOXEL_CASES)
 def test_voxel_filter_against_the_reference_build(orc, n, voxel, seed):
-    """The REFERENCE's own CFilter::voxelfilter (include/filter.hpp compiled verbatim, build container only): same number of
+    """The REFERENCE's own CFilter::voxelfilter (include/filter.hpp compiled verbatim; its outputs are stored): same number of
     output points, the phantom point 0 first, the same voxel at every output position.  WHICH point of a voxel is kept is
     implementation-defined there (an unstable std::sort on the voxel id alone, :71); the oracle / CUDA path keep the smallest
     index."""
     P = scan_like_cloud(n, seed)
-    ref = orc.ref_voxelfilter(P, voxel)
-    if ref is None:
-        pytest.skip("oracle/_ref/libprep_ref.so not built (no /root/reference here)")
+    ref = P[rg.load("voxel")[rg.key(n, voxel, seed)]]          # stored as the rows of P the reference kept
     mine = P[orc.voxel_downsample(P, voxel)]
     assert len(ref) == len(mine)
     assert np.array_equal(ref[0], P[0]) and np.array_equal(mine[0], P[0])
@@ -63,17 +67,15 @@ def test_voxel_filter_against_the_reference_build(orc, n, voxel, seed):
     assert np.array_equal(vr[1:], vm[1:])                      # same voxel, position by position (position 0 is the phantom)
 
 
-@pytest.mark.parametrize("n,radius,nms,seed", [(4000, 1.0, 1.5, 8), (1500, 0.6, 0.6, 9), (600, 3.0, 0.3, 10), (6000, 0.8, 1.0, 12)])
+@pytest.mark.parametrize("n,radius,nms,seed", KEYPOINT_CASES)
 def test_keypoint_detection_against_the_reference_build(orc, n, radius, nms, seed):
     """The REFERENCE's own keypointDetectionBasedOnCurvature (keypoint_detect.hpp + pca.h compiled verbatim: its PCA driver,
     pruneUnstablePoints, the curvature sort and the std::set based greedy suppression; KD-tree / PCA numerics from the
-    stand-ins): normally the same number of keypoints with the same curvature at every output position, indices differing
-    only between points of EXACTLY equal curvature that suppress each other — the reference orders such ties through an
-    unstable std::sort (:151), the oracle / CUDA path by index."""
+    stand-ins; its outputs are stored): normally the same number of keypoints with the same curvature at every output
+    position, indices differing only between points of EXACTLY equal curvature that suppress each other — the reference
+    orders such ties through an unstable std::sort (:151), the oracle / CUDA path by index."""
     P = scan_like_cloud(n, seed)
-    ref = orc.ref_detect_keypoints(P, radius, 0.65, 20, nms)
-    if ref is None:
-        pytest.skip("oracle/_ref/libprep_ref.so not built (no /root/reference here)")
+    ref = rg.load("keypoints")[rg.key(n, radius, nms, seed)]
     kp, lam, curv, cnt = orc.detect_keypoints(P, radius, 0.65, 20, nms)
     assert len(kp) > 0
     if np.array_equal(curv[ref], curv[kp]):
